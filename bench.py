@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- sliding-window solves/sec on synthetic 10-frame x 150-feature windows (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); the windows are independent, so the batch is split across ranks
 with no data-path collective (weak scaling: 1024 windows per GPU) and NCCL is only used for the barrier and the
@@ -16,6 +16,9 @@ dogleg iterations) over one batch of 1024 windows per GPU.
   --impl reference : the CPU path (oracle port of the reference's Ceres solve; the reference itself cannot be
           compiled here) on all host cores over the same 1024-window batch per step.
 Inputs per step (about 340 MB per GPU) are larger than the 126 MB L2, so no explicit L2 flush is needed.
+  --dump-outputs DIR : after the timed steps, what each timed path returned in its last step (solved states and solve
+          reports, float64; every window, or a fixed seeded sample of them past 64 MB) as DIR/{resident,e2e}_<name>.npy, so
+          that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -25,6 +28,8 @@ import sys
 import threading
 import time
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -32,6 +37,7 @@ WINDOWS_PER_GPU = 1024
 FEATURES = 150
 PRIOR_FEATURES = 24
 CPU_SAMPLE = 256
+DUMP_LIMIT = 64 << 20          # bytes of --dump-outputs in all; beyond it a fixed seeded sample of windows
 
 
 def static_config(NW, F, world):
@@ -83,6 +89,29 @@ class ClockSampler:
                 if v.lower().startswith("active"):
                     reasons.add(name)
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None, "reasons": sorted(reasons), "samples": len(self.rows)}
+
+
+def solve_outputs(batch, rep):
+    """What a caller of the solve receives for each window: the solved states and the solve report, as float64."""
+    st = batch.state_array()
+    out = {k: st[k].astype(np.float64) for k in st.dtype.names}
+    out["para_Feature"] = batch.para_Feature.copy()
+    for k in rep.dtype.names:
+        out["report_" + k] = rep[k].astype(np.float64)
+    return out
+
+
+def dump_outputs(directory, prefix, outputs, limit):
+    """directory/<prefix><name>.npy for every output, rows = windows; over `limit` bytes, a fixed seeded sample of the windows
+    (their indices in <prefix>window_index.npy either way)."""
+    os.makedirs(directory, exist_ok=True)
+    n = len(next(iter(outputs.values())))
+    per_window = 8 + sum(a.nbytes for a in outputs.values()) / n
+    keep = min(n, int(limit // per_window))
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    np.save(os.path.join(directory, prefix + "window_index.npy"), idx.astype(np.float64))
+    for k, a in outputs.items():
+        np.save(os.path.join(directory, prefix + k + ".npy"), a[idx])
 
 
 def usable_cpus():
@@ -187,6 +216,7 @@ def main():
     ap.add_argument("--features", type=int, default=FEATURES)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--distinct", type=int, default=0, help="distinct synthetic windows to generate (tiled up to --windows); 0: all distinct up to 200 features, else 64")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the outputs of the last timed step of each path to DIR/*.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -195,7 +225,6 @@ def main():
         run_reference(args, rank, world)
         return
 
-    import numpy as np
     from cerberus_b200 import abi, synth, lib, parallel
     dist = None
     device = None
@@ -241,6 +270,8 @@ def main():
             ev_ms += ms; launches += nl
         wall_resident = time.perf_counter() - t0
         barrier()
+        if args.dump_outputs:                            # the resident path's last step, fetched outside the timed region
+            resident_out = solve_outputs(batch, gpu.download(batch))
         # ---- end to end through the host-buffer call ---------------------------------------------------------------
         e2e_s = 0.0
         regs = gpu.register_batch(batch)                 # page-lock the caller's arrays once (outside the timed region)
@@ -256,6 +287,10 @@ def main():
         e2e_ms, e2e_launches = gpu.last_solve_stats()
         gpu.unregister(regs)
     clocks = clk.summary()
+    if args.dump_outputs:
+        tag = f"rank{rank}_" if world > 1 else ""
+        dump_outputs(args.dump_outputs, tag + "resident_", resident_out, DUMP_LIMIT // (2 * world))
+        dump_outputs(args.dump_outputs, tag + "e2e_", solve_outputs(batch, rep), DUMP_LIMIT // (2 * world))
     if dist is not None:
         ev_ms = parallel.max_over_ranks(ev_ms, dist, device)
         e2e_s = parallel.max_over_ranks(e2e_s, dist, device)

@@ -82,13 +82,13 @@ def test_bad_descriptors_are_rejected():
 
 def test_integration_stub_compiles_against_the_header_and_reference_headers():
     """tools/integration_stub.cpp (the reference-side binding of INTEGRATION.md) type-checks as C++14 against include/cerberus_b200.h, the
-    reference's own headers where they lie and the Eigen / ROS / OpenCV shims of oracle/shim; the header alone also compiles as plain C."""
+    reference's own headers (where `make -C oracle ref` finds the reference's sources: oracle/Makefile's REF; the repository does not carry
+    them) and the Eigen / ROS / OpenCV shims of oracle/shim; the header alone also compiles as plain C."""
     hdr_c = subprocess.run(["gcc", "-std=c99", "-fsyntax-only", "-x", "c", os.path.join(ROOT, "include", "cerberus_b200.h")], capture_output=True, text=True)
     assert hdr_c.returncode == 0, hdr_c.stderr
-    if not os.path.isdir("/root/reference/src"):
-        pytest.skip("/root/reference absent (GPU box)")
-    r = subprocess.run(["g++", "-std=c++14", "-fsyntax-only", "-w", "-I" + os.path.join(ROOT, "include"), "-I" + os.path.join(ROOT, "oracle", "shim"),
-                        "-I/root/reference/src", os.path.join(ROOT, "tools", "integration_stub.cpp")], capture_output=True, text=True)
+    r = subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "stub-check"], capture_output=True, text=True)
+    if "reference sources not present" in r.stdout:
+        pytest.skip("the reference's sources are not present (oracle/Makefile REF)")
     assert r.returncode == 0, r.stderr[-3000:]
 
 

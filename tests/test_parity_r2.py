@@ -3,7 +3,8 @@
 CPU tier (`-m "not gpu"`):
   * cerb_double2vector (the gauge re-anchoring of Estimator::double2vector, estimator.cpp:903-957 -- the function that produces the
     poses the estimator publishes) against the oracle restatement AND against the reference's own Utility::R2ypr / ypr2R
-    (utils/utility.cpp compiled into oracle/_ref), including the singular-pitch branch (:925-934);
+    (utils/utility.cpp compiled into oracle/_ref, outputs recorded in tests/golden/ref_v1.npz), including the singular-pitch
+    branch (:925-934);
   * the per-feature steps (triangulate / outlier errors / depth shift) of the oracle and of the kernels (CPU simulator) against
     the reference's own FeatureManager (featureTracker/feature_manager.cpp compiled into oracle/_ref) and the statements of
     Estimator::reprojectionError / outliersRejection executed over it.
@@ -14,12 +15,12 @@ import os
 import numpy as np
 import pytest
 from cerberus_b200 import abi, synth, lib
-from oracle_lib import OracleBackend, RefBackend, ref_lib
+from oracle_lib import OracleBackend
+from ref_golden import reference
 from helpers import sim_backend, small_cfg, prior_canonical, state_diffs, SIM_LIB
 from test_preintegration import make_jobs
 
 ob = OracleBackend()
-needs_ref = pytest.mark.skipif(ref_lib() is None, reason="oracle/_ref not built and /root/reference absent")
 
 
 # ---------------------------------------------------------------------------------------------------- double2vector
@@ -60,12 +61,12 @@ D2V_PITCHES = [(5.0, -7.0), (30.0, 29.0), (-45.0, -44.0), (89.6, 20.0), (10.0, -
 
 def _check_d2v(cdll):
     rng = np.random.default_rng(12)
-    ref = RefBackend() if ref_lib() is not None else None
+    ref = reference()
     singular = 0
     for (pb, pa) in D2V_PITCHES * 3:
         before, after = _d2v_states(rng, pb, pa)
         got = _d2v_product(cdll, before, after)
-        for arm in ([ob] if ref is None else [ob, ref]):
+        for arm in (ob, ref):
             want = arm.double2vector(before, after)
             for g, w, name in zip(got, want, ("Ps", "Rs", "Vs")):
                 assert np.abs(g - w).max() < 1e-12 * max(1.0, np.abs(w).max()), (name, pb, pa, type(arm).__name__)
@@ -78,12 +79,10 @@ def _check_d2v(cdll):
     assert singular >= 9
 
 
-@needs_ref
 def test_double2vector_sim_build_vs_oracle_and_reference():
     _check_d2v(C.CDLL(SIM_LIB) if os.path.exists(SIM_LIB) else sim_backend(small_cfg()).lib)
 
 
-@needs_ref
 def test_double2vector_product_library_vs_oracle_and_reference():
     """The sm_100a library's host-side cerb_double2vector (no device involved: callable without a GPU)."""
     if not os.path.exists(lib.PRODUCT_LIB):
@@ -96,14 +95,41 @@ def test_double2vector_product_library_vs_oracle_and_reference():
 
 
 # ---------------------------------------------------------------------------------------------------- n3 against reference source
-@needs_ref
+def _feature_steps_vs_reference(be, ref, realistic):
+    """The kernels' outlier errors, depth shift and triangulation against the reference's FeatureManager on fixed inputs: the initial
+    states, the states the oracle solves to, and the latter with every second feature not triangulated (estimated_depth = -1)."""
+    from test_feature_steps import _batch
+    batch = _batch(ob, realistic)
+    nf = [batch.descs[w].n_features for w in range(batch.n)]
+    for phase in range(3):
+        if phase == 1:
+            OracleBackend(small_cfg(max_batch=4, max_features=24, iters=3)).solve_batch(batch)
+        if phase == 2:
+            for w in range(batch.n):
+                batch.para_Feature[w, 0:nf[w]:2] = -1.0
+        be.upload(batch)
+        err, rem = be.outlier_errors(batch.n); e_ref = ref.outlier_errors(batch)
+        st_g, dep_g, keep_g = be.shift_depth(batch.n, 7.5); st_r, dep_r, keep_r = ref.shift_depth(batch, 7.5)
+        dep = be.triangulate(batch.n); t_ref = ref.triangulate(batch)
+        for w in range(batch.n):
+            k = nf[w]
+            if phase < 2:
+                ok = np.isfinite(e_ref[w, :k])       # the reference skips used_num < 4 (estimator.cpp:1750)
+                assert ok.sum() >= k - 1 and np.abs(err[w, :k][ok] - e_ref[w, :k][ok]).max() < 1e-12 * max(1.0, np.abs(e_ref[w, :k][ok]).max())
+                assert (rem[w, :k][ok] == (e_ref[w, :k][ok] * 460.0 > 3)).all()
+            kp = keep_r[w, :k] != 0
+            assert (keep_g[w, :k] == keep_r[w, :k]).all() and (st_g[w, :k][kp] == st_r[w, :k][kp]).all()
+            assert np.abs(dep_g[w, :k][kp] - dep_r[w, :k][kp]).max() < 1e-12 * np.abs(dep_r[w, :k][kp]).max()
+            assert np.abs(dep[w, :k] - t_ref[w, :k]).max() < 1e-8 * np.abs(t_ref[w, :k]).max()
+
+
 @pytest.mark.parametrize("realistic", [False, True])
 def test_feature_steps_oracle_and_sim_vs_reference_feature_manager(realistic):
     """FeatureManager::{triangulate, triangulatePoint, removeBackShiftDepth} (feature_manager.cpp:198-212,302-385,450-488) and the
     statements of Estimator::{reprojectionError, outliersRejection} (estimator.cpp:1729-1798) executed from the reference's source."""
-    from test_feature_steps import _check_backend, _batch
+    from test_feature_steps import _batch
     cfg = small_cfg(max_batch=4, max_features=24, iters=3)
-    ref = RefBackend()
+    ref = reference()
     # oracle restatement vs reference source
     batch = _batch(ob, realistic)
     nf = [batch.descs[w].n_features for w in range(batch.n)]
@@ -123,8 +149,8 @@ def test_feature_steps_oracle_and_sim_vs_reference_feature_manager(realistic):
             keep = s1[2][w, :k] != 0
             assert (s0[0][w, :k][keep] == s1[0][w, :k][keep]).all() and (s0[2][w, :k] == s1[2][w, :k]).all()
             assert np.abs(s0[1][w, :k][keep] - s1[1][w, :k][keep]).max() < 1e-12 * np.abs(s1[1][w, :k][keep]).max()
-    # kernels (CPU simulator) vs reference source
-    _check_backend(sim_backend(cfg), ref, realistic)
+    # kernels (CPU simulator) vs reference source; the simulator against the oracle through the whole sequence: test_feature_steps.py
+    _feature_steps_vs_reference(sim_backend(cfg), ref, realistic)
 
 
 # ---------------------------------------------------------------------------------------------------- GPU tier
@@ -134,8 +160,6 @@ def _gpu(cfg=None):
 
 @pytest.mark.gpu
 def test_double2vector_product_library_gpu_box():
-    ref_ok = ref_lib() is not None
-    assert ref_ok, "oracle/_ref/libcerberus_ref.so travels with the snapshot"
     _check_d2v(_gpu().lib)
 
 
@@ -145,7 +169,7 @@ def test_imu_preintegration_and_imu_factor_gpu():
     integration_base.h / imu_factor.h (oracle/_ref)."""
     from test_reference_pin import imu_setup
     gpu = _gpu()
-    arms = [ob] + ([RefBackend()] if ref_lib() is not None else [])
+    arms = [ob, reference()]
     jobs, _, _ = make_jobs(6, seed=29)
     pcfg = abi.default_preint_config()
     got = gpu.preintegrate_imu(pcfg, jobs, 6)
@@ -173,16 +197,11 @@ def test_imu_preintegration_and_imu_factor_gpu():
 @pytest.mark.gpu
 def test_prior_evaluator_gpu():
     """cerb_eval_prior (MarginalizationFactor::Evaluate, marginalization_factor.cpp:347-395) on the device vs oracle and reference."""
+    from test_reference_pin import prior_probe
     gpu = _gpu()
-    batch = synth.generate_batch(1, 8, ob, prior_features=6)
-    st = batch.state_array()
-    st["para_Pose"][0, :, :3] += 0.02; st["para_SpeedBias"][0, 0] += 0.01; st["para_LegBias"][0, 0] += 1e-3
-    st["para_Pose"][0, :, 3:7] += 0.003; st["para_Pose"][0, :, 3:7] /= np.linalg.norm(st["para_Pose"][0, :, 3:7], axis=-1, keepdims=True)
-    st["para_Pose"][0, 2, 3:7] *= -1.0                       # w < 0 branch of the rotation residual (:369-375)
-    pr = batch.descs[0].prior
-    ncols = 7 * 12 + 9 + 4 + 1
+    batch, pr, ncols = prior_probe()
     r1, j1 = gpu.eval_prior(pr, batch.states[0], ncols)
-    for arm in [ob] + ([RefBackend()] if ref_lib() is not None else []):
+    for arm in (ob, reference()):
         r0, j0 = arm.eval_prior(pr, batch.states[0], ncols)
         assert np.abs(r0 - r1).max() < 1e-10 * np.abs(r0).max() and np.abs(j0 - j1).max() == 0.0
 
@@ -213,7 +232,7 @@ def test_marginalization_with_prior_gpu(margin_old):
     gpu = lib.Backend(cfg)
     mk = lambda: synth.generate_batch(2, 10, ob, with_prior=True, window0=47)
     src = mk()
-    arms = [ob] + ([RefBackend()] if ref_lib() is not None else [])
+    arms = [ob, reference()]
     c = mk(); gpu.marginalize(cfg, src, c, margin_old)
     for arm in arms:
         a = mk(); arm.marginalize(cfg, src, a, margin_old)
@@ -227,10 +246,8 @@ def test_marginalization_with_prior_gpu(margin_old):
 @pytest.mark.gpu
 @pytest.mark.parametrize("realistic", [False, True])
 def test_feature_steps_gpu_vs_reference_feature_manager(realistic):
-    from test_feature_steps import _check_backend
-    assert ref_lib() is not None
     cfg = small_cfg(max_batch=4, max_features=24, iters=4)
-    _check_backend(lib.Backend(cfg), RefBackend(), realistic)
+    _feature_steps_vs_reference(lib.Backend(cfg), reference(), realistic)
 
 
 @pytest.mark.gpu
